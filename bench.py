@@ -7,6 +7,7 @@
     python bench.py --impl reference ...      # BASELINE config 1 on the box's host cores: HTTP-dispatched CPU workers
     python bench.py --workload img2img        # BASELINE config 3
     python bench.py --sweep 1,2,4,8,16,32,64  # BASELINE config 5 (per-GPU batch sweep), one JSON line with a list
+    python bench.py --dump-outputs DIR        # also write the last timed step's images to DIR as .npy, to compare builds
 
 One "step" = one whole txt2img request of the per-GPU batch: CLIP encode, 20 DDIM timesteps (19 UNet evaluations
 on [cond | uncond]) and the VAE decode to uint8, plus — for N > 1 — the single NCCL all-gather of the images.
@@ -413,6 +414,23 @@ def synthetic_inputs(eng, b, rank):
     return tokens, neg, seed0, x_T, init_u8
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out_dir, images):
+    """images [n, H, W, 3] uint8 -> out_dir/images.npy float32 (values 0..255) and out_dir/images_index.npy float64 (their
+    indices in the batch).  Whole images are kept, as many as fit DUMP_BYTES, chosen by a fixed seed, so that two builds
+    run with the same arguments write the same images and can be compared value for value."""
+    import numpy as np
+    n = images.shape[0]
+    per_image = images[0].numel() * 4 + 8
+    keep = min(n, (DUMP_BYTES - 1024) // per_image)   # 1024: the two .npy headers
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "images.npy"), images.cpu()[idx].float().numpy())
+    np.save(os.path.join(out_dir, "images_index.npy"), idx.double().numpy())
+
+
 def make_step(eng, workload, b, tokens_d, neg_d, x_T_d, init_d, seed0, world, gather):
     """one request with its inputs already on the device: conditioning, sampling, VAE decode (+ the all-gather)"""
     from b200sd import engine as E
@@ -428,7 +446,7 @@ def make_step(eng, workload, b, tokens_d, neg_d, x_T_d, init_d, seed0, world, ga
         lat = eng.run_program(cond, unc, pr.start(x_T_d, init), pr, CFG_SCALE, noises=draws)
         u8 = eng.decode(lat, HW, HW)
         if world > 1:
-            gather(u8, [b] * world)
+            u8 = gather(u8, [b] * world)
         return u8
 
     return step
@@ -436,7 +454,8 @@ def make_step(eng, workload, b, tokens_d, neg_d, x_T_d, init_d, seed0, world, ga
 
 def timed_device(eng, step, steps, warmup, barrier, rank, local, world, dev):
     """W >= 3 untimed requests, then exactly K timed ones between barrier + synchronize on both sides; CUDA events, max
-    over ranks.  Returns (ms, clocks during the timed region, b200sd kernels launched inside it)."""
+    over ranks.  Returns (ms, clocks during the timed region, b200sd kernels launched inside it, the last timed step's
+    images)."""
     import torch.distributed as dist
     from b200sd import ops
     for _ in range(max(3, warmup)):
@@ -450,7 +469,7 @@ def timed_device(eng, step, steps, warmup, barrier, rank, local, world, dev):
     l0 = ops.LAUNCHES + eng.graph_replayed_launches
     e0.record()
     for _ in range(steps):
-        step()
+        out = step()
     e1.record()
     barrier()
     launches = ops.LAUNCHES + eng.graph_replayed_launches - l0
@@ -459,7 +478,7 @@ def timed_device(eng, step, steps, warmup, barrier, rank, local, world, dev):
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    return float(t.item()), clk, launches
+    return float(t.item()), clk, launches, out
 
 
 # ================================================================================================ main
@@ -479,9 +498,16 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-world", action="store_true")
     ap.add_argument("--no-stock", action="store_true")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the images of the last timed step to DIR/images.npy (float32; a seeded sample of whole "
+                         "images when the batch exceeds 64 MB) and their batch indices to DIR/images_index.npy")
     ap.add_argument("--serve-cpu-oracle", type=int, default=None, help=argparse.SUPPRESS)
     ap.add_argument("--threads", type=int, default=0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.sweep or args.impl == "reference"):
+        ap.error("--dump-outputs applies to the main measurement of --impl b200, not to --sweep or --impl reference")
     if args.serve_cpu_oracle is not None:
         return serve_cpu_oracle(args.serve_cpu_oracle, args.threads or usable_cpus(), args.model)
     rank, world, local = dist_env()
@@ -546,7 +572,7 @@ def main():
             tk, ng, sd0, xt, iu8 = synthetic_inputs(eng, bb, rank)
             step = make_step(eng, args.workload, bb, tk.to(dev), ng.to(dev), xt.to(dev), iu8.to(dev), sd0, world,
                              all_gather_images)
-            ms, ck, _ = timed_device(eng, step, args.steps, args.warmup, barrier, rank, local, world, dev)
+            ms, ck, _, _ = timed_device(eng, step, args.steps, args.warmup, barrier, rank, local, world, dev)
             rows.append({"per_gpu_batch": bb, "global_batch": bb * world, "value": world * bb * args.steps / (ms / 1000.0),
                          "ms_per_step": ms / args.steps, "clocks": ck})
             eng.plans.pop((bb, HW, HW), None)
@@ -571,8 +597,11 @@ def main():
     tokens, neg, seed0, x_T, init_u8 = synthetic_inputs(eng, b, rank)
     step_device = make_step(eng, args.workload, b, tokens.to(dev), neg.to(dev), x_T.to(dev), init_u8.to(dev), seed0, world,
                             all_gather_images)
-    elapsed_ms, clk, gpu_launches = timed_device(eng, step_device, args.steps, args.warmup, barrier, rank, local, world, dev)
+    elapsed_ms, clk, gpu_launches, images = timed_device(eng, step_device, args.steps, args.warmup, barrier, rank, local,
+                                                         world, dev)
     value = world * b * args.steps / (elapsed_ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, images)
 
     # ---------------- e2e through the plugin surface (host buffers, H2D + D2H inside the timed region), one world per rank
     e2e = None

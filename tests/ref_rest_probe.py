@@ -1,9 +1,9 @@
-"""Drives a running sdwui-API worker server with the UNMODIFIED reference `Worker` class (/root/reference), in its own
-process because the reference's module names (`scripts.spartan.*`) are the same as this repo's.
+"""Drives a running sdwui-API worker server with the UNMODIFIED reference `Worker` class, in its own process because the
+reference's module names (`scripts.spartan.*`) are the same as this repo's.
 
-    python tests/ref_rest_probe.py <port>        -> one JSON line on stdout
+    python tests/ref_rest_probe.py <port> <reference checkout>       -> one JSON line on stdout
 
-Used by tests/test_rest_worker_cpu.py when /root/reference exists (build container only).
+Used by tests/golden/gen_rest_worker_golden.py.
 """
 import base64
 import io
@@ -14,7 +14,7 @@ import sys
 import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("REFERENCE_DIR", "/root/reference")
+REF = sys.argv[2]
 tmp = tempfile.mkdtemp(prefix="refprobe_")
 os.environ["HOSTSTUB_CONFIG_DIR"] = tmp
 sys.path[:0] = [os.path.join(HERE, "hoststub"), REF]

@@ -1,6 +1,7 @@
 """SURVEY §8 row f1: the sdwui-compatible REST worker (server/sdapi.py), driven over real HTTP by
  (1) this repo's `Worker` (which keeps the reference's HTTP transport for remote nodes), and
- (2) the UNMODIFIED reference `Worker` in a subprocess, when /root/reference exists (build container only).
+ (2) the UNMODIFIED reference `Worker`: the requests it sent and what it made of the replies are stored golden data
+     (tests/golden/gen_rest_worker_golden.py -> tests/golden/rest_worker_golden.json), replayed here over HTTP.
 The executor is replaced by a deterministic double: this file tests the wire contract, not the arithmetic."""
 import base64
 import hashlib
@@ -8,8 +9,6 @@ import io
 import json
 import os
 import socket
-import subprocess
-import sys
 import threading
 import time
 import types
@@ -19,6 +18,7 @@ import pytest
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+REST_GOLDEN = os.path.join(HERE, "golden", "rest_worker_golden.json")
 
 
 class EngineDouble:
@@ -79,6 +79,17 @@ def server():
 def _decode(b64png):
     from PIL import Image
     return np.asarray(Image.open(io.BytesIO(base64.b64decode(b64png))))
+
+
+def reply_digest(path, body):
+    """what the REST golden file keeps of a reply: images as the SHA-1 of their decoded pixels, and of /memory (live
+    numbers, and 'cuda' depends on the machine) only whether the fields the reference Worker reads are there"""
+    if path.endswith("/memory"):
+        cuda = body.get("cuda", {})
+        return {"keys": sorted(body), "cuda_readable": "error" in cuda or {"free", "total"} <= set(cuda.get("system", {}))}
+    if isinstance(body, dict) and "images" in body:
+        return dict(body, images=[hashlib.sha1(_decode(s).tobytes()).hexdigest() for s in body["images"]])
+    return body
 
 
 PAYLOAD = {"prompt": "a probe", "negative_prompt": "", "seed": 31, "subseed": 7, "subseed_strength": 0, "batch_size": 2,
@@ -205,15 +216,20 @@ def test_requests_are_bounded_and_restart_waits_for_the_running_generation():
     assert evicted == [True]            # the restart ran after the generation had been released
 
 
-@pytest.mark.skipif(not os.path.isdir(os.environ.get("REFERENCE_DIR", "/root/reference")),
-                    reason="the unmodified reference exists in the build container only")
 def test_unmodified_reference_worker_drives_the_rest_server(server):
+    """the requests the reference Worker sent, replayed: the server answers each as it did when the reference drove it,
+    so the reference would reach the same state and images it did then"""
     port, eng = server
-    p = subprocess.run([sys.executable, os.path.join(HERE, "ref_rest_probe.py"), str(port)], capture_output=True, text=True,
-                       timeout=120)
-    assert p.returncode == 0, p.stderr[-2000:]
-    out = json.loads(p.stdout.strip().splitlines()[-1])
-    assert out["reference_file"].startswith(os.environ.get("REFERENCE_DIR", "/root/reference"))
+    import requests
+    with open(REST_GOLDEN) as f:
+        golden = json.load(f)
+    assert [e["path"].rsplit("/", 1)[1] for e in golden["exchange"]] == ["memory", "memory", "options", "txt2img", "sd-models"]
+    for e in golden["exchange"]:
+        r = requests.request(e["method"], f"http://127.0.0.1:{port}{e['path']}", json=e["json"], timeout=30)
+        assert r.status_code == e["status"], e["path"]
+        assert reply_digest(e["path"], r.json()) == e["reply"], e["path"]
+    assert eng.calls[-1] == ("txt2img", 31, 2, 4, "DDIM")
+    out = golden["reference_worker"]
     assert out["reachable"] and out["state"] == "IDLE" and out["n_images"] == 2
     assert out["all_seeds"] == [31, 32] and out["all_subseeds"] == [7, 8]
     want = _expected(eng, PAYLOAD)
